@@ -7,6 +7,7 @@ random-init weights (seed 0), fp16 tensor-core compute.  Metric = input megapixe
 
   python bench.py --gpus N --steps K --warmup W            # this repo's engine (one rank per GPU under torchrun)
   python bench.py --impl reference ...                      # the reference algorithm on the host CPU cores (oracle port)
+  python bench.py --dump-outputs DIR ...                    # also write the last timed step's output to DIR/*.npy
 
 One JSON line is printed by rank 0.  See DESIGN.md "Measurement" for every field.
 """
@@ -39,6 +40,28 @@ IW3_WORKLOADS = {
                        text="iw3 ZoeD_N (BEiT-L) + dilate_edge 2 + backward (grid_sample) warp + dubois anaglyph, 4K stream (configs[4])"),
 }
 SWIN4X_TILE_GFLOP = 155.7           # BASELINE.md section 2 (conv 8.6 + addmm 140.1 + bmm 7.0)
+# --dump-outputs keeps at most this many float32 values in all (32 MiB): the 4K swin4x output alone is 4e8 values (1.6 GB)
+DUMP_ELEMS = 1 << 23
+
+
+def dump_outputs(path, outputs, seed=0):
+    """Write each output tensor as <path>/<name>.npy in float32: whole if it fits its share of DUMP_ELEMS, otherwise that many
+    flat elements at sorted indices drawn from a generator seeded with `seed`, so two runs with the same arguments (two builds
+    of the project) dump the same positions.  Returns {name: {"shape": full shape, "dumped": elements written}}."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    share = DUMP_ELEMS // len(outputs)
+    info = {}
+    for name, t in outputs.items():
+        if t.numel() > share:
+            idx = torch.randint(t.numel(), (share,), generator=torch.Generator().manual_seed(seed)).sort().values
+            a = t.reshape(-1)[idx.to(t.device)]
+        else:
+            a = t
+        np.save(os.path.join(path, name + ".npy"), a.float().cpu().numpy())
+        info[name] = {"shape": list(t.shape), "dumped": a.numel()}
+    return info
 
 
 def load_peaks():
@@ -626,6 +649,7 @@ def run_b200_iw3(args):
         launches = lib.nb200_launch_count() - launches0
         ms = e0.elapsed_time(e1)
         out_shape = list(y.shape)
+        dumped = dump_outputs(args.dump_outputs, {"stereo_frames": y}) if args.dump_outputs and rank == 0 else None
     # ---- end to end from host uint8 frames (outside inference_mode: the pipeline enters it around the callback itself)
     u8_in = (c.permute(0, 2, 3, 1) * 255.0).round().to(torch.uint8).contiguous().cpu().pin_memory()   # contiguous HWC, like a decoder's frame
     frames_host = [u8_in[i] for i in range(B)]
@@ -701,6 +725,8 @@ def run_b200_iw3(args):
         "gpu_launches": int(launches), "clocks": clocks.summary(), "roofline": roof,
         "kernel_classes_ms": {k: round(v["ms"], 4) for k, v in prof.items()},
     }
+    if dumped:
+        line["dump_outputs"] = dumped
     if rank == 0:
         if world == 1 and not args.no_cpu_baseline:
             try:
@@ -775,7 +801,7 @@ def run_b200(args):
     with torch.no_grad():
         for _ in range(args.warmup):
             y = step()
-        del y
+        y = None
         barrier()
         launches0 = lib.nb200_launch_count()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -787,6 +813,7 @@ def run_b200(args):
             barrier()
         launches = lib.nb200_launch_count() - launches0
         ms = e0.elapsed_time(e1)
+        dumped = dump_outputs(args.dump_outputs, {"output": y}) if args.dump_outputs and rank == 0 else None
         del y
         # ---- end-to-end through the public API with host buffers (H2D + render + D2H every step)
         e2e_steps = max(1, min(args.steps, 3))
@@ -901,6 +928,8 @@ def run_b200(args):
         line["swin_downscaled2x_8k"] = cfg4
     if iw3 is not None:
         line["iw3_1080p"] = iw3
+    if dumped:
+        line["dump_outputs"] = dumped
     if rank == 0:
         if world == 1 and not args.no_cpu_baseline:
             line["cpu_baseline"] = guarded(lambda: cpu_baseline_object(h, w, ntiles)[1])
@@ -920,7 +949,14 @@ def main():
     ap.add_argument("--frame", default=None, choices=list(FRAME), help="frame size (default: the workload's)")
     ap.add_argument("--workload", default="swin4x_4k", choices=list(WORKLOADS) + list(IW3_WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="--impl b200: after the timed steps, write the last step's output to DIR/<name>.npy (float32; a fixed "
+                         "seeded sample of it when it exceeds 32 MiB)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs is implemented for --impl b200")
     if args.cpu_worker:
         cpu_worker_main(*args.cpu_worker)
     elif args.workload in IW3_WORKLOADS:

@@ -421,9 +421,19 @@ def gen_zoedepth_infer():
     save("zoedepth_infer", **out)
 
 
+def gen_transformers():
+    """transformers' Depth-Anything-V2 and ZoeDepth models, the independent implementations the depth-network oracles are
+    pinned to, on the seeded cases of tests/test_oracle_golden.py: the pin then holds without transformers installed."""
+    import transformers
+    from tests import test_oracle_golden as tog
+    save("transformers_depth", depth_anything=tog.hf_depth_anything(*tog.da_case()), zoedepth=tog.hf_zoedepth(*tog.zoe_case()),
+         transformers_version=np.asarray(transformers.__version__))
+
+
 if __name__ == "__main__":
     os.makedirs(OUT, exist_ok=True)
-    which = sys.argv[1:] or ["seam", "models", "iw3", "alpha_tta", "frames", "row_flow", "row_flow_steps", "postprocess", "depth_scaler", "depth_aa", "mlbw", "mlbw_variants", "zoedepth_infer"]
+    which = sys.argv[1:] or ["seam", "models", "iw3", "alpha_tta", "frames", "row_flow", "row_flow_steps", "postprocess", "depth_scaler",
+                             "depth_aa", "mlbw", "mlbw_variants", "zoedepth_infer", "transformers"]
     if "seam" in which:
         gen_seam_config()
     if "models" in which:
@@ -450,3 +460,5 @@ if __name__ == "__main__":
         gen_mlbw_variants()
     if "zoedepth_infer" in which:
         gen_zoedepth_infer()
+    if "transformers" in which:
+        gen_transformers()

@@ -1,5 +1,6 @@
 """Pin the CPU oracle to the committed outputs of the real reference
 (tests/golden/*.npz, produced by oracle/gen_golden.py).  CPU only."""
+import importlib.util
 import os
 import numpy as np
 import pytest
@@ -247,14 +248,20 @@ def _da_to_hf(sd, depth=12):
     return out
 
 
-def test_depth_anything_oracle_matches_transformers():
-    """The Depth-Anything-V2 network is third-party code absent from /root/reference (torch.hub).  Pin the oracle's
-    restatement against the independent public implementation in this image (transformers), same weights."""
-    transformers = pytest.importorskip("transformers")
+DA_GRID = 6
+
+
+def da_case():
+    """(weights, input) of the Depth-Anything-V2 comparison with transformers."""
+    sd = synth.depth_anything_v2_state_dict(3, pos_grid=DA_GRID)
+    x = torch.randn(2, 3, 14 * DA_GRID, 14 * DA_GRID, generator=torch.Generator().manual_seed(5))
+    return sd, x
+
+
+def hf_depth_anything(sd, x):
+    """transformers.DepthAnythingForDepthEstimation loaded with the oracle's weights: predicted depth for x."""
     from transformers import DepthAnythingConfig, DepthAnythingForDepthEstimation, Dinov2Config
-    from oracle import depth_anything as oda
-    grid = 6
-    sd = synth.depth_anything_v2_state_dict(3, pos_grid=grid)
+    grid = DA_GRID
     cfg = DepthAnythingConfig(
         backbone_config=Dinov2Config(hidden_size=384, num_hidden_layers=12, num_attention_heads=6, mlp_ratio=4, image_size=14 * grid,
                                      patch_size=14, out_features=["stage3", "stage6", "stage9", "stage12"],
@@ -264,13 +271,30 @@ def test_depth_anything_oracle_matches_transformers():
     hf = DepthAnythingForDepthEstimation(cfg).eval()
     missing, unexpected = hf.load_state_dict(_da_to_hf(sd), strict=False)
     assert not unexpected and all("position_ids" in m or "rel" in m for m in missing), (missing, unexpected)
-    x = torch.randn(2, 3, 14 * grid, 14 * grid, generator=torch.Generator().manual_seed(5))
     with torch.no_grad():
-        want = hf(pixel_values=x).predicted_depth
+        return hf(pixel_values=x).predicted_depth
+
+
+def transformers_wants(key, fn, *args):
+    """What transformers computes for a case: the output stored in tests/golden/transformers_depth.npz (oracle/gen_golden.py
+    transformers), so the pin holds where the package is not installed, plus a fresh run where it is."""
+    wants = [t(load("transformers_depth")[key])]
+    if importlib.util.find_spec("transformers") is not None:
+        wants.append(fn(*args))
+    return wants
+
+
+def test_depth_anything_oracle_matches_transformers():
+    """The Depth-Anything-V2 network is third-party code that the reference fetches through torch.hub.  Pin the oracle's
+    restatement against an independent public implementation (transformers), same weights."""
+    from oracle import depth_anything as oda
+    sd, x = da_case()
+    with torch.no_grad():
         got = oda.depth_anything_forward(sd, x)
-    assert got.shape == want.shape == (2, 14 * grid, 14 * grid)
-    assert float(want.std()) > 0.1
-    assert float((got - want).abs().max()) < 2e-4 * float(want.abs().max())
+    for want in transformers_wants("depth_anything", hf_depth_anything, sd, x):
+        assert got.shape == want.shape == (2, 14 * DA_GRID, 14 * DA_GRID)
+        assert float(want.std()) > 0.1
+        assert float((got - want).abs().max()) < 2e-4 * float(want.abs().max())
 
 
 def test_zoe_preprocess_oracle_matches_reference():
@@ -473,15 +497,18 @@ def _zoe_to_hf(sd, cfg):
     return out
 
 
-def test_zoedepth_oracle_matches_transformers():
-    """ZoeD_N (BEiT-L + DPT + metric bins) is third-party code absent from /root/reference (torch.hub).  Pin the oracle's
-    restatement against the independent public implementation in this image (transformers), same weights, on a
-    non-square input so that the relative-position table is resampled."""
-    pytest.importorskip("transformers")
+def zoe_case():
+    """(weights, input) of the ZoeD_N comparison with transformers: non-square, so the relative-position table is resampled."""
+    sd = synth.zoedepth_state_dict(3, synth.ZOED_MINI)
+    x = torch.randn(2, 3, 64, 96, generator=torch.Generator().manual_seed(5))
+    return sd, x
+
+
+def hf_zoedepth(sd, x):
+    """transformers.ZoeDepthForDepthEstimation at the reduced widths of ZOED_MINI, loaded with the oracle's weights."""
     from transformers import ZoeDepthConfig, ZoeDepthForDepthEstimation, BeitConfig
     from oracle import zoedepth as oz
     cfg = oz.ZOED_MINI
-    sd = synth.zoedepth_state_dict(3, synth.ZOED_MINI)
     hf_cfg = ZoeDepthConfig(
         backbone_config=BeitConfig(image_size=16 * cfg["old_grid"], patch_size=16, hidden_size=cfg["dim"], num_hidden_layers=cfg["depth"],
                                    num_attention_heads=cfg["heads"], intermediate_size=4 * cfg["dim"], use_relative_position_bias=True,
@@ -494,13 +521,22 @@ def test_zoedepth_oracle_matches_transformers():
     hf = ZoeDepthForDepthEstimation(hf_cfg).eval()
     missing, unexpected = hf.load_state_dict(_zoe_to_hf(sd, cfg), strict=False)
     assert not unexpected and all("relative_position_index" in m or "k_idx" in m or "k_minus_1" in m for m in missing), (missing, unexpected)
-    x = torch.randn(2, 3, 64, 96, generator=torch.Generator().manual_seed(5))
     with torch.no_grad():
-        want = hf(pixel_values=x).predicted_depth
-        got = oz.zoedepth_forward(sd, x, cfg)[:, 0]
-    assert got.shape == want.shape == (2, 64, 96)
-    assert float(want.std()) > 0.05
-    assert float((got - want).abs().max()) < 2e-4 * float(want.abs().max())
+        return hf(pixel_values=x).predicted_depth
+
+
+def test_zoedepth_oracle_matches_transformers():
+    """ZoeD_N (BEiT-L + DPT + metric bins) is third-party code that the reference fetches through torch.hub.  Pin the oracle's
+    restatement against an independent public implementation (transformers), same weights, on a non-square input so that
+    the relative-position table is resampled."""
+    from oracle import zoedepth as oz
+    sd, x = zoe_case()
+    with torch.no_grad():
+        got = oz.zoedepth_forward(sd, x, oz.ZOED_MINI)[:, 0]
+    for want in transformers_wants("zoedepth", hf_zoedepth, sd, x):
+        assert got.shape == want.shape == (2, 64, 96)
+        assert float(want.std()) > 0.05
+        assert float((got - want).abs().max()) < 2e-4 * float(want.abs().max())
 
 
 def test_zoedepth_batch_infer_oracle_matches_reference():
