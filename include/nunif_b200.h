@@ -339,6 +339,36 @@ int nb200_profile_enable(int on);
 int nb200_profile_report(char* buf, size_t cap);
 int nb200_profile_dump(char* buf, size_t cap);   /* one CSV line per timed launch: class,ms,work,read_bytes,write_bytes */
 
+/* ------------------------------------------------------------------ *
+ * Low-level ops of the depth networks, exposed for unit tests
+ * (csrc/depth_kernels.cu, csrc/zoe_kernels.cu; the Depth-Anything-V2 and
+ * ZoeD_N forwards above are sequences of these and the GEMM)
+ * ------------------------------------------------------------------ */
+
+/* dinov2 Attention / BEiT attention core: softmax(q k^T / 8 [+ bias]) v per image and head, head dim 64.
+ * qkv fp16 [B*N][3*heads*64] (q | k | v, head-major) -> out fp16 [B*N][heads*64].  bias_log2e (may be NULL): fp32
+ * [heads][N][ldb] already multiplied by log2 e, shared by the B images; ldb even and >= cdiv(N, 64) * 64. */
+int nb200_vit_attention_f16(const void* qkv, void* out, int B, int N, int heads, const float* bias_log2e, int ldb,
+                            void* stream);
+/* residual add + LayerNorm(eps=1e-6) of the ViT blocks: x32 fp32 [rows][dim] += fp16 delta (may be NULL);
+ * out fp16 [rows][dim] = LayerNorm(x32) * w + b (out NULL: only the residual is updated).  dim in {256, 384, 768, 1024}. */
+int nb200_vit_add_layernorm(float* x32, const void* delta, const float* w, const float* b, void* out, long long rows,
+                            int dim, void* stream);
+/* MiDaS beit.py gen_relative_position_index gather: bias[h][q][k] (row stride ldb >= N, N = ph*pw + 1) =
+ * table[index(q, k)][h] * log2 e; table fp32 [(2ph-1)(2pw-1) + 3][heads].  Columns [N, ldb) are not written. */
+int nb200_zoe_expand_rel_bias(const float* table, int ph, int pw, int heads, float* bias, int ldb, void* stream);
+/* ZoeDepth AttractorLayerUnnormed (softplus attractors, align-corners bilinear prev_bin, inv_attractor mean):
+ * apre fp16 [B*H*W][lda] (first na used), prev_bin fp32 [B][h][w][64] -> out fp32 [B][H][W][64]. */
+int nb200_zoe_attractor(const void* apre, int lda, int na, const float* prev_bin, int B, int h, int w, int H, int W,
+                        float* out, void* stream);
+/* ZoeDepth ConditionalLogBinomial tail + sum_k prob_k * centre_k: g fp16 [B*H*W][ldg >= 80] (GELU'd hidden), w2 fp32
+ * [4][80], b2 [4], bins fp32 [B][h][w][64] (align-corners bilinear to H x W) -> depth fp32 [B][H][W]. */
+int nb200_zoe_clb_final(const void* g, int ldg, const float* w2, const float* b2, const float* bins, int B, int h, int w,
+                        int H, int W, float* depth, void* stream);
+/* F.interpolate(x, (H, W), mode="bilinear", align_corners=True) of the DPT head on fp16 NHWC:
+ * x [B][h][w][C] -> out [B][H][W][C], C % 8 == 0. */
+int nb200_dpt_upsample_bilinear_f16(const void* x, int B, int h, int w, int C, void* out, int H, int W, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -107,6 +107,13 @@ SIGNATURES = {
     "nb200_swin_attn_tc_f16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int,
                                        c_void_p]),
     "nb200_window_attention_f16": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),
+    "nb200_vit_attention_f16": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_void_p]),
+    "nb200_vit_add_layernorm": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, ctypes.c_longlong, c_int, c_void_p]),
+    "nb200_zoe_expand_rel_bias": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_void_p]),
+    "nb200_zoe_attractor": (c_int, [c_void_p, c_int, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
+    "nb200_zoe_clb_final": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p,
+                                    c_void_p]),
+    "nb200_dpt_upsample_bilinear_f16": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_int, c_int, c_void_p]),
 }
 
 

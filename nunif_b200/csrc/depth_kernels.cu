@@ -478,3 +478,26 @@ int da_head_final(cudaStream_t st, const __half* x, long long npix, int C, const
 }
 
 }  // namespace nb200
+
+using namespace nb200;
+
+// Low-level ops of the depth networks exposed for unit tests (see include/nunif_b200.h).
+extern "C" int nb200_vit_attention_f16(const void* qkv, void* out, int B, int N, int heads, const float* bias_log2e, int ldb,
+                                       void* stream) {
+    NB_CHECK(qkv && out, "null pointer");
+    NB_CHECK(B >= 1 && N >= 1 && heads >= 1, "empty attention");
+    return da_attention((cudaStream_t)stream, (const __half*)qkv, (__half*)out, B, N, heads, bias_log2e, ldb);
+}
+
+extern "C" int nb200_vit_add_layernorm(float* x32, const void* delta, const float* w, const float* b, void* out, long long rows,
+                                       int dim, void* stream) {
+    NB_CHECK(x32 && (!out || (w && b)), "null pointer");
+    NB_CHECK(rows >= 1, "empty input");
+    return da_add_layernorm((cudaStream_t)stream, x32, (const __half*)delta, w, b, (__half*)out, rows, dim);
+}
+
+extern "C" int nb200_dpt_upsample_bilinear_f16(const void* x, int B, int h, int w, int C, void* out, int H, int W, void* stream) {
+    NB_CHECK(x && out, "null pointer");
+    NB_CHECK(B >= 1 && h >= 1 && w >= 1 && H >= 1 && W >= 1, "empty image");
+    return da_upsample_bilinear((cudaStream_t)stream, (const __half*)x, B, h, w, C, (__half*)out, H, W);
+}

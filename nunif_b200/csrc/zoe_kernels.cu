@@ -376,3 +376,26 @@ int zoe_clb_final(cudaStream_t st, const __half* g, int ldg, const float* w2, co
 }
 
 }  // namespace nb200
+
+using namespace nb200;
+
+// Low-level ops of the depth networks exposed for unit tests (see include/nunif_b200.h).
+extern "C" int nb200_zoe_expand_rel_bias(const float* table, int ph, int pw, int heads, float* bias, int ldb, void* stream) {
+    NB_CHECK(table && bias, "null pointer");
+    NB_CHECK(ph >= 1 && pw >= 1 && heads >= 1, "empty token grid");
+    return zoe_expand_rel_bias((cudaStream_t)stream, table, ph, pw, heads, bias, ldb);
+}
+
+extern "C" int nb200_zoe_attractor(const void* apre, int lda, int na, const float* prev_bin, int B, int h, int w, int H, int W,
+                                   float* out, void* stream) {
+    NB_CHECK(apre && prev_bin && out, "null pointer");
+    NB_CHECK(B >= 1 && h >= 1 && w >= 1 && H >= 1 && W >= 1, "empty image");
+    return zoe_attractor((cudaStream_t)stream, (const __half*)apre, lda, na, prev_bin, B, h, w, H, W, out);
+}
+
+extern "C" int nb200_zoe_clb_final(const void* g, int ldg, const float* w2, const float* b2, const float* bins, int B, int h, int w,
+                                   int H, int W, float* depth, void* stream) {
+    NB_CHECK(g && w2 && b2 && bins && depth, "null pointer");
+    NB_CHECK(B >= 1 && h >= 1 && w >= 1 && H >= 1 && W >= 1, "empty image");
+    return zoe_clb_final((cudaStream_t)stream, (const __half*)g, ldg, w2, b2, bins, B, h, w, H, W, depth);
+}
